@@ -21,12 +21,16 @@ through NCCL is timed beside it at N > 1).
 
 Timing: W warm-up steps, then a barrier + synchronize, then the timed steps with one CUDA event
 per step on the engine's stream, then the exchange stream joined, a final event, barrier +
-synchronize.  The timed region runs --steps K steps or --min-time seconds of device time, whichever
-is MORE (a 30 ms region cannot be timed across 8 ranks); `steps` in the line is what ran,
-`steps_requested` what was asked.  MAX over ranks.  Clocks are sampled through NVML inside the
-process (no nvidia-smi subprocess between the barrier and the first step).
+synchronize.  With --steps K the timed region runs exactly K steps.  Without it, it runs 200 steps
+or --min-time seconds of device time (default 1 s), whichever is MORE (a 30 ms region cannot be
+timed across 8 ranks); giving both makes --min-time a floor on top of K.  `steps` in the line is
+what ran, `steps_requested` what was asked.  MAX over ranks.  Clocks are sampled through NVML
+inside the process (no nvidia-smi subprocess between the barrier and the first step).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+--dump-outputs DIR writes what the last timed step computed (rank 0) as DIR/<name>.npy, float64,
+so that two builds can be compared output for output on the same seeded snapshot: see dump_outputs.
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -391,6 +395,33 @@ def step_stats(per):
             "max_ms": float(per.max()), "mean_ms": float(per.mean())}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_PODS = 256
+
+
+def dump_outputs(eng, out_dir):
+    """Writes the round the engine last evaluated as its caller receives it: every decision vector of bs_fetch in
+    full, and the rows of a fixed, seeded sample of pods (`pod_sample`) of the P x N score matrix and of the fit
+    bitmap (words), which are GB-sized at the headline size.  float64 holds every value exactly: scores are small
+    integers or INT64_MIN ("no fit"), the rest are 32-bit integers."""
+    res = eng.fetch()
+    arrays = {f: getattr(res, f) for f in ("prefilter", "feasible_count", "best_node", "best_score", "admit",
+                                           "admit_bitmap", "new_denied", "order", "rank")}
+    arrays["max_group"] = np.array([res.max_group])
+    arrays["max_finished"] = np.array([res.max_finished])
+    rng = np.random.default_rng(0)
+    pods = np.sort(rng.choice(eng.P, min(eng.P, DUMP_SAMPLE_PODS), replace=False))
+    arrays["pod_sample"] = pods
+    arrays["score_rows"] = np.concatenate([eng.score_rows(int(p), 1) for p in pods])
+    arrays["fit_bitmap_rows"] = np.concatenate([eng.fit_rows(int(p), 1) for p in pods])
+    total = sum(a.size * 8 for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total / 2**20:.0f} MB (limit 64 MB); use a smaller --scale")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def make_nccl_exchange(H, eng, capi):
     """all_gather_into_tensor over a torch view of the engine's admit-bitmap device buffer, enqueued on
     the engine's stream right behind the round."""
@@ -521,8 +552,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=None)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scale", type=float, default=1.0, help="shrink the workload (debug only; marks the line)")
-    ap.add_argument("--min-time", type=float, default=1.0,
-                    help="the timed region lasts at least this many seconds of device time (more steps than --steps if needed)")
+    ap.add_argument("--min-time", type=float, default=None,
+                    help="the timed region lasts at least this many seconds of device time (more steps than --steps if "
+                         "needed); default 1 s without --steps, none with it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-replay", action="store_true", help="skip the multi-round admission leg")
     ap.add_argument("--no-strong", action="store_true", help="N>1: skip the strong-scaling legs")
@@ -530,6 +564,8 @@ def main():
     ap.add_argument("--exchange", default="both", choices=["p2p", "nccl", "both"],
                     help="N>1: admit-bitmap all-gather by the engine's peer-memory kernels (headline), by NCCL, or both")
     args = ap.parse_args()
+    if args.min_time is None:
+        args.min_time = 0.0 if args.steps is not None else 1.0
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -603,6 +639,8 @@ def main():
         launches_per_step = None
     head_key = "p2p" if use_p2p else ("single" if world == 1 else "nccl")
     head = legs[head_key]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     total_pairs = H.sum_over_ranks(float(P) * N)
     total_groups = H.sum_over_ranks(float(G))
     value = total_pairs * head["steps"] / (head["ms_total"] * 1e-3)

@@ -1,4 +1,4 @@
-import sys,time,importlib; sys.path.insert(0,'/root/repo')
+import sys,time,importlib,os; sys.path.insert(0,os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 pkg=importlib.import_module("batch-scheduler_b200")
 import numpy as np
 S=pkg.snapshot
