@@ -3,8 +3,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <type_traits>
-
 #include "../../include/bsched.h"
 
 namespace bsk {
@@ -45,59 +43,19 @@ struct LaneMap {
   uint32_t sclamp[BS_MAX_LANES]; // C = 2^(28-k), or 1 when k > 28
   uint32_t LW, LN, LS;
 };
-#ifndef BS_FIT_TILE
-#define BS_FIT_TILE 512
-#endif
-constexpr int NODE_TILE = BS_FIT_TILE;                  // nodes per shared-memory tile (128 / 256 / 512 / 1024)
-#ifndef BS_FIT_WARPS
-#define BS_FIT_WARPS 8
-#endif
-#ifndef BS_FIT_PPW
-#define BS_FIT_PPW 4
-#endif
-constexpr int FIT_WARPS = BS_FIT_WARPS;                 // consumer warps (each sweeps PODS_PER_WARP pods)
+constexpr int NODE_TILE = 512;                          // nodes per shared-memory tile
+constexpr int FIT_WARPS = 8;                            // consumer warps (each sweeps PODS_PER_WARP pods)
 constexpr int FIT_THREADS = (FIT_WARPS + 1) * 32;       // + one producer warp that only drives the TMA ring
-constexpr int PODS_PER_WARP = BS_FIT_PPW;               // pods evaluated together per node (ILP)
+constexpr int PODS_PER_WARP = 4;                        // pods evaluated together per node (ILP)
 constexpr int PODS_PER_CTA = FIT_WARPS * PODS_PER_WARP; // 32
 constexpr int TILE_WORDS = NODE_TILE / 32;              // ballot words per tile and pod
 static_assert(TILE_WORDS <= 32 && 32 % TILE_WORDS == 0, "a 32-word bitmap line is a whole number of tiles");
 constexpr int TILES_PER_LINE = 32 / TILE_WORDS;         // tiles whose ballot words fill one 128-byte bitmap line
-constexpr int KEY_BITS = TILE_WORDS <= 2 ? 1 : TILE_WORDS <= 4 ? 2 : TILE_WORDS <= 8 ? 3 : 4;   // log2(TILE_WORDS)
-static_assert(TILE_WORDS <= 16, "best-node key: score (27 bits) + word index (4 bits) must fit 31 bits");
-#ifndef BS_FIT_STAGES
-#define BS_FIT_STAGES 2
-#endif
-constexpr int FIT_STAGES = BS_FIT_STAGES;               // TMA ring depth (full/empty mbarrier pairs)
-// Score rows leave the SMs with 8-byte streaming stores (BS_FIT_STG, default).  -DBS_FIT_TMA_STORE stages them in
-// shared memory and hands FIT_SEG-node row segments to the TMA engine instead (cp.async.bulk shared -> global):
-// built, parity-tested and measured in round 2 — 3 % slower in the kernel (the per-segment proxy fence and
-// issue cost more than the cleaner HBM burst pattern returns), see profiles/README.md.
-#if !defined(BS_FIT_TMA_STORE) && !defined(BS_FIT_STG)
-#define BS_FIT_STG 1
-#endif
-#ifndef BS_FIT_SEG
-#ifdef BS_FIT_STG
-#define BS_FIT_SEG BS_FIT_TILE
-#else
-#define BS_FIT_SEG 128
-#endif
-#endif
-constexpr int FIT_SEG = BS_FIT_SEG;                     // nodes per score store segment (one bulk store per pod row)
-constexpr int SEG_WORDS = FIT_SEG / 32;
-static_assert(NODE_TILE % FIT_SEG == 0 && FIT_SEG % 128 == 0, "a tile is a whole number of 128-node-multiple segments");
-#ifndef BS_FIT_NB
-#define BS_FIT_NB 2
-#endif
-constexpr int FIT_NB = BS_FIT_NB;                       // score staging slabs (segments) per warp in flight
+constexpr int KEY_BITS = 4;                             // log2(TILE_WORDS): score (27 bits) + word index fit 31 bits
+static_assert(TILE_WORDS == 1 << KEY_BITS, "best-node key: KEY_BITS is log2(TILE_WORDS)");
+constexpr int FIT_STAGES = 2;                           // TMA ring depth (full/empty mbarrier pairs)
 // class bits of the TILE_WORDS nodes a lane owns in one tile
-using ColBits = std::conditional<(TILE_WORDS > 32), uint64_t,
-                                 std::conditional<(TILE_WORDS > 16), uint32_t,
-                                                  std::conditional<(TILE_WORDS > 8), uint16_t, uint8_t>::type>::type>::type;
-#ifndef BS_FIT_MINB
-#define BS_FIT_MINB 2
-#endif
-#ifndef BS_FIT_MINB_NOSCORE
-#define BS_FIT_MINB_NOSCORE 2
-#endif
+using ColBits = uint16_t;
+static_assert(sizeof(ColBits) * 8 == TILE_WORDS, "ColBits holds one bit per node a lane owns in a tile");
 
 }  // namespace bsk

@@ -234,8 +234,6 @@ struct bs_engine {
   // trailing zeros = the power of two every value is a multiple of) and max |residual|
   uint64_t or_left[BS_MAX_LANES] = {}, or_req[BS_MAX_LANES] = {};
   int64_t max_left[BS_MAX_LANES] = {};
-  int exp_mode = 0;                     // BS_EXP_MODE (measurement experiments only): 1 skip the sort, 2 fit after sort + chain, 3 skip the chain's overlap
-  bool no_scaled_lanes = false;         // BS_NO_SCALED_LANES=1: keep byte-valued lanes in int64 (experiments)
   uint32_t score_pitch = 0;             // elements per score row: N rounded up to even
   uint32_t bitmap_pitch = 0;            // words per fit-bitmap row: ceil(N/32) rounded up to 32 (whole 128-byte lines)
   // pod table
@@ -654,7 +652,7 @@ LaneMap classify_lanes(const bs_engine* e) {
     const int64_t mx = std::max(e->max_left[d], e->max_req[d]);
     uint32_t k_need = 0;
     while (k_need < 63 && (mx >> k_need) > SCALED_LIMIT) ++k_need;
-    if (k_need <= k_avail && !e->no_scaled_lanes) {
+    if (k_need <= k_avail) {
       kind[d] = SCALED;
       unit[d] = k_need;
       ++ls;
@@ -947,7 +945,7 @@ int evaluate_async_locked(bs_engine* e) {
   {
     StageTimer tm(e, BS_K_SORT, e->s2);
     // one persistent kernel: group keys -> sort -> dense group rank -> pod keys -> sort -> order + rank
-    if ((P || G) && e->exp_mode != 1) {
+    if (P || G) {
       SortArgs sa{};
       sa.creation = e->d_creation.as<int64_t>();
       sa.name_rank = e->d_name_rank.as<uint32_t>();
@@ -1055,8 +1053,6 @@ int evaluate_async_locked(bs_engine* e) {
     }
   }
   CK(cudaEventRecord(e->ev_pre, e->s3));
-  if (e->exp_mode == 2) { CK(cudaStreamWaitEvent(e->s, e->ev_join, 0)); CK(cudaStreamWaitEvent(e->s, e->ev_pre, 0)); }
-  if (e->exp_mode == 3) CK(cudaStreamWaitEvent(e->s, e->ev_pre, 0));
   {
     StageTimer tm(e, BS_K_GANG_FIT, e->s, true);
     if (P) {
@@ -1252,8 +1248,6 @@ int bs_create(const bs_config* cfg, bs_engine** out) {
   e->device = cfg->device;
   e->L = cfg->n_lanes;
   e->out_flags = cfg->out_flags;
-  if (const char* ns = getenv("BS_NO_SCALED_LANES")) e->no_scaled_lanes = atoi(ns) != 0;
-  if (const char* xm = getenv("BS_EXP_MODE")) e->exp_mode = atoi(xm);
   e->host_prof = getenv("BS_HOST_PROFILE") != nullptr;
   int prio_lo = 0, prio_hi = 0;
   cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // the small kernels of the PreFilter chain must get the

@@ -3,9 +3,6 @@
 // fit_lookup()).
 #pragma once
 #include "common.cuh"
-#ifndef BS_FIT_EXP
-#define BS_FIT_EXP 0   // 0 = product; 1 / 2 = store-path experiments (profiles/README.md), never shipped
-#endif
 
 namespace bsk {
 
@@ -24,14 +21,11 @@ namespace bsk {
 //   INPUT: the producer lane streams the tiles of the residual table into a FIT_STAGES-deep
 //     shared-memory ring with 1-D TMA bulk copies (cp.async.bulk global->shared, one per lane
 //     row), guarded by full/empty mbarrier pairs; consumers never meet at a CTA-wide barrier.
-//   OUTPUT (round 2): score rows do NOT leave through the LSU.  A warp writes the NODE_TILE
-//     scores of each of its pods into a private staging slab in shared memory (st.shared.u64,
-//     conflict-free) and one lane hands every row segment — NODE_TILE*8 contiguous bytes of one
-//     matrix row — to the TMA engine (cp.async.bulk shared->global, bulk_group completion);
-//     FIT_NB slabs per warp rotate, a slab is refilled once its bulk reads have finished
-//     (cp.async.bulk.wait_group.read).  HBM then sees 2 KB bursts per row instead of 256-byte
-//     pieces of four interleaved rows: the store pattern alone went from 1.34 ms to 1.14 ms for
-//     the 8 GB matrix of the bench workload (profiles/microbench/store_pattern2.cu; cudaMemset 1.09).
+//   OUTPUT: each lane writes the score of every pair it evaluates straight from registers with an
+//     8-byte streaming store (st.global.cs, SASS STG.E.EF.64): 256 contiguous bytes of one matrix
+//     row per warp store.  Ballot words are assembled in a per-warp shared-memory slab and leave as
+//     one aligned 128-byte bitmap line per pod and 1024 nodes.  Staging the scores in shared memory
+//     for TMA bulk stores was measured 3 % slower in the kernel (DESIGN §4, profiles/README.md).
 // A lane owns nodes lane, lane+32, ... of the tile, keeps their `left` in registers and evaluates
 // PODS_PER_WARP pods against them at a time.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -68,26 +62,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst_smem, const void* src_gme
       "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
       : "memory");
 }
-// shared -> global bulk store (TMA), completion tracked by the issuing thread's bulk async-group
-__device__ __forceinline__ void tma_bulk_s2g(void* dst_gmem, uint32_t src_smem, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem), "r"(src_smem), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ uint64_t l2_evict_first_policy() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void tma_bulk_s2g_hint(void* dst_gmem, uint32_t src_smem, uint32_t bytes, uint64_t pol) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst_gmem), "r"(src_smem),
-               "r"(bytes), "l"(pol)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-// generic-proxy shared-memory writes -> visible to the async proxy (the TMA engine reads the slab)
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 __device__ __forceinline__ int64_t min64(int64_t a, int64_t b) { return a < b ? a : b; }
 // high word of an int64, opaque to the optimiser (it otherwise re-forms a 2-instruction 64-bit compare)
@@ -103,17 +77,11 @@ __device__ __forceinline__ uint32_t lo32(int64_t v) {
   (void)hi;
   return (uint32_t)lo;
 }
-// Shared-memory stores of the hot loop.  volatile (never dropped, kept in order among themselves) but
-// WITHOUT a "memory" clobber: the compiler may hoist the next nodes' LDS above them (the slabs they write
-// are only read after a __syncwarp / fence, which are compiler barriers).
+// Ballot-word store of the hot loop.  volatile (never dropped, kept in order among themselves) but
+// WITHOUT a "memory" clobber: the compiler may hoist the next nodes' LDS above it (the slab it writes
+// is only read after a __syncwarp, which is a compiler barrier).
 __device__ __forceinline__ void sts_u32(uint32_t saddr, uint32_t v) {
   asm volatile("st.shared.u32 [%0], %1;" ::"r"(saddr), "r"(v));
-}
-__device__ __forceinline__ void sts_v2u32(uint32_t saddr, uint32_t lo, uint32_t hi) {
-  asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(saddr), "r"(lo), "r"(hi));
-}
-__device__ __forceinline__ void sts_u64(uint32_t saddr, long long v) {
-  asm volatile("st.shared.u64 [%0], %1;" ::"r"(saddr), "l"(v));
 }
 
 struct FitArgs {
@@ -134,7 +102,7 @@ struct FitArgs {
   // form of `int32 base + (uint32 Npad << 2)` (a lone ULEA with the high word zeroed) when the
   // TMA source address of a narrow row is derived from a 32-bit Npad; 64-bit pitches avoid it.
   uint64_t left_w_pitch, left_n_pitch;
-  uint64_t score_pitch;   // elements per score row: N rounded up to even (16-byte row starts for the bulk stores)
+  uint64_t score_pitch;   // elements per score row: N rounded up to even (16-byte row starts)
   uint32_t bitmap_pitch;  // words per fit-bitmap row: ceil(N/32) rounded up to 32 (rows are whole 128-byte lines)
   uint32_t P, N, Npad, W;
   // Tail balance: CTA units (PODS_PER_CTA pods x the whole node range) [0, n_full) fill whole waves of the
@@ -156,31 +124,29 @@ template <> struct BestT<true> { using type = int32_t; };
 //     joins the fit test, x << k (exact original units, or 2^27 = "cannot be the minimum") joins the min;
 //   wide lanes: 64-bit subtract, sign through the high word, low word when the high word is 0.
 // Ballot words go to a per-warp shared-memory slab (one STS per pair, every lane writes the same word);
-// scores go to the warp's staging slab (SCORE) as int64: fit ? m : INT64_MIN.
+// scores (SCORE) go to rows row0 .. row0 + PODS_PER_WARP - 1 of the matrix as int64: fit ? m : INT64_MIN.
 // OUT: what leaves the SMs besides the per-pod results — 0 nothing (decisions only: feasible counts come from a
 // predicated add, no ballot), 1 the fit bitmap, 2 the score matrix (+ the bitmap when its pointer is set).
 enum { FIT_OUT_NONE = 0, FIT_OUT_BITMAP = 1, FIT_OUT_SCORE = 2 };
 template <int LW, int LN, int LS, int OUT>
-__device__ __forceinline__ void fit_seg(const FitArgs& a, const int64_t* __restrict__ tlw,
-                                         const int32_t* __restrict__ tln,
-                                         const int64_t (&rqw)[PODS_PER_WARP][LW > 0 ? LW : 1],
-                                         const int32_t (&rqn)[PODS_PER_WARP][LN + LS > 0 ? LN + LS : 1],
-                                         const ColBits (&colbits)[PODS_PER_WARP], uint32_t slab /*smem addr*/,
-                                         uint32_t* s_words, uint32_t wbase /*tile's first word in the line*/, uint32_t node_base, uint32_t lane,
-                                         int j0 /*first word of the segment*/,
-                                         typename BestT<(LN > 0)>::type (&best_s)[PODS_PER_WARP],
-                                         int32_t (&best_n)[PODS_PER_WARP], int32_t (&kb)[PODS_PER_WARP],
-                                         uint32_t (&cnt)[PODS_PER_WARP], uint32_t stg_row0 = 0) {
+__device__ __forceinline__ void fit_tile(const FitArgs& a, const int64_t* __restrict__ tlw,
+                                          const int32_t* __restrict__ tln,
+                                          const int64_t (&rqw)[PODS_PER_WARP][LW > 0 ? LW : 1],
+                                          const int32_t (&rqn)[PODS_PER_WARP][LN + LS > 0 ? LN + LS : 1],
+                                          const ColBits (&colbits)[PODS_PER_WARP],
+                                          uint32_t* s_words, uint32_t wbase /*tile's first word in the line*/, uint32_t node_base, uint32_t lane,
+                                          typename BestT<(LN > 0)>::type (&best_s)[PODS_PER_WARP],
+                                          int32_t (&best_n)[PODS_PER_WARP], int32_t (&kb)[PODS_PER_WARP],
+                                          uint32_t (&cnt)[PODS_PER_WARP], uint32_t row0) {
   constexpr bool SCORE = OUT == FIT_OUT_SCORE;
   constexpr bool WORDS = OUT != FIT_OUT_NONE;
-  const int64_t* tpw = tlw + lane + j0 * 32;
-  const int32_t* tpn = tln + lane + j0 * 32;
-  int32_t node = (int32_t)(node_base + lane) + j0 * 32;
-  uint32_t wp = smem_u32(s_words) + (wbase + j0) * 4;   // word (wbase + j) of the 32-word line being assembled
-  uint32_t sp = slab + lane * 8;
-  int32_t jrem = TILE_WORDS - 1 - j0;   // best-node key: low KEY_BITS bits = TILE_WORDS-1-j (earlier node wins a tie)
+  const int64_t* tpw = tlw + lane;
+  const int32_t* tpn = tln + lane;
+  int32_t node = (int32_t)(node_base + lane);
+  uint32_t wp = smem_u32(s_words) + wbase * 4;   // word (wbase + j) of the 32-word line being assembled
+  int32_t jrem = TILE_WORDS - 1;   // best-node key: low KEY_BITS bits = TILE_WORDS-1-j (earlier node wins a tie)
 #pragma unroll 1
-  for (int jb = j0; jb < j0 + SEG_WORDS; jb += 4) {
+  for (int jb = 0; jb < TILE_WORDS; jb += 4) {
 #pragma unroll
     for (int jj = 0; jj < 4; ++jj) {
       int64_t lfw[LW > 0 ? LW : 1];
@@ -191,11 +157,6 @@ __device__ __forceinline__ void fit_seg(const FitArgs& a, const int64_t* __restr
       for (int d = 0; d < LN + LS; ++d) lfn[d] = tpn[d * NODE_TILE + jj * 32];
 #pragma unroll
       for (int r = 0; r < PODS_PER_WARP; ++r) {
-#if BS_FIT_EXP >= 3    // (experiments 3-5: no arithmetic at all, the store structure alone)
-        if (SCORE) sts_v2u32(sp + (r * FIT_SEG + jj * 32) * 8, (uint32_t)node, 0u);
-        sts_u32(wp + (r * 32 + jj) * 4, 0xffffffffu);
-        continue;
-#endif
         if (LN > 0) {
           // Narrow fast path.  t = min over the narrow lanes is a REAL difference (the narrow set
           // holds a fixed lane) with |t| < 2^27, and the pair's score m = min over all lanes <= t.
@@ -226,13 +187,9 @@ __device__ __forceinline__ void fit_seg(const FitArgs& a, const int64_t* __restr
           // (scores of fitting pairs are < 2^27), -1 = none; decoded once per tile
           const int32_t key = (int32_t)(m32 << KEY_BITS) + (jrem - jj);
           if (fit) kb[r] = max(kb[r], key);
-#ifdef BS_FIT_STG     // (experiment: scores straight to HBM with 8-byte streaming stores, no staging / TMA)
           if (SCORE && (uint32_t)(node + jj * 32) < a.N)
-            __stcs(reinterpret_cast<unsigned long long*>(a.score) + (size_t)(stg_row0 + r) * a.score_pitch + (node + jj * 32),
+            __stcs(reinterpret_cast<unsigned long long*>(a.score) + (size_t)(row0 + r) * a.score_pitch + (node + jj * 32),
                    (unsigned long long)(fit ? m32 : 0u) | ((unsigned long long)(fit ? 0u : 0x80000000u) << 32));
-#elif BS_FIT_EXP != 2   // (experiment 2: bulk stores without the staging stores)
-          if (SCORE) sts_v2u32(sp + (r * FIT_SEG + jj * 32) * 8, fit ? m32 : 0u, fit ? 0u : 0x80000000u);
-#endif
         } else {
           int64_t m = lfw[0] - rqw[r][0];
 #pragma unroll
@@ -241,13 +198,9 @@ __device__ __forceinline__ void fit_seg(const FitArgs& a, const int64_t* __restr
           if (WORDS) sts_u32(wp + (r * 32 + jj) * 4, __ballot_sync(0xffffffffu, fit));
           else if (fit) ++cnt[r];
           if (fit && m > best_s[r]) { best_s[r] = m; best_n[r] = node + jj * 32; }
-#ifdef BS_FIT_STG
           if (SCORE && (uint32_t)(node + jj * 32) < a.N)
-            __stcs(reinterpret_cast<long long*>(a.score) + (size_t)(stg_row0 + r) * a.score_pitch + (node + jj * 32),
+            __stcs(reinterpret_cast<long long*>(a.score) + (size_t)(row0 + r) * a.score_pitch + (node + jj * 32),
                    fit ? (long long)m : (long long)INT64_MIN);
-#else
-          if (SCORE) sts_u64(sp + (r * FIT_SEG + jj * 32) * 8, fit ? (long long)m : (long long)INT64_MIN);
-#endif
         }
       }
     }
@@ -256,53 +209,37 @@ __device__ __forceinline__ void fit_seg(const FitArgs& a, const int64_t* __restr
     node += 128;
     jrem -= 4;
     wp += 16;
-    sp += 128 * 8;
   }
 }
 
 __host__ __device__ constexpr size_t fit_tile_bytes(int LW, int LN, int LS) {
   return (size_t)NODE_TILE * (8 * LW + 4 * (LN + LS));
 }
-__host__ __device__ constexpr size_t fit_slab_bytes() { return (size_t)PODS_PER_WARP * FIT_SEG * 8; }
-// shared-memory layout: [stages]{[LW][NODE_TILE] i64, [LN+LS][NODE_TILE] i32} | req_w | req_n | mbarriers |
-//                       ballot words | (SCORE) [FIT_WARPS][FIT_NB] staging slabs, 128-byte aligned
-__host__ __device__ constexpr size_t fit_smem_front(int LW, int LN, int LS, int stages) {
-  size_t b = stages * fit_tile_bytes(LW, LN, LS) + (size_t)PODS_PER_CTA * (8 * LW + 4 * (LN + LS));
+// shared-memory layout: [FIT_STAGES]{[LW][NODE_TILE] i64, [LN+LS][NODE_TILE] i32} | req_w | req_n | mbarriers |
+//                       ballot words, 128-byte aligned
+__host__ __device__ constexpr size_t gang_fit_smem_bytes(int LW, int LN, int LS) {
+  size_t b = FIT_STAGES * fit_tile_bytes(LW, LN, LS) + (size_t)PODS_PER_CTA * (8 * LW + 4 * (LN + LS));
   b = (b + 7) & ~(size_t)7;
-  b += 2 * stages * sizeof(uint64_t) + (size_t)PODS_PER_CTA * 32 * sizeof(uint32_t);
+  b += 2 * FIT_STAGES * sizeof(uint64_t) + (size_t)PODS_PER_CTA * 32 * sizeof(uint32_t);
   return (b + 127) & ~(size_t)127;
 }
-__host__ __device__ constexpr size_t fit_smem_total(int LW, int LN, int LS, bool score, int stages) {
-  return fit_smem_front(LW, LN, LS, stages) + (score ? (size_t)FIT_WARPS * FIT_NB * fit_slab_bytes() : 0);
-}
-// input ring depth: FIT_STAGES where the CTA's shared memory allows it (227 KB per CTA on sm_100a), else 2
-constexpr size_t FIT_SMEM_MAX = 227 * 1024;
-__host__ __device__ constexpr int fit_stages(int LW, int LN, int LS, bool score) {
-  return fit_smem_total(LW, LN, LS, score, FIT_STAGES) <= FIT_SMEM_MAX ? FIT_STAGES : 2;
-}
-inline size_t gang_fit_smem_bytes(int LW, int LN, int LS, bool score) {
-#ifdef BS_FIT_STG
-  score = false;   // no staging slabs
-#endif
-  return fit_smem_total(LW, LN, LS, score, fit_stages(LW, LN, LS, score));
-}
+// the widest shape (every lane wide) must fit the 227 KB a CTA may have on sm_100a
+static_assert(gang_fit_smem_bytes(BS_MAX_LANES, 0, 0) <= 227 * 1024, "gang_fit_kernel: shared memory over 227 KB");
 
 template <int LW, int LN, int LS, int OUT>
-__global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MINB : BS_FIT_MINB_NOSCORE) gang_fit_kernel(FitArgs a) {
-  constexpr bool SCORE = OUT == FIT_OUT_SCORE;
+__global__ void __launch_bounds__(FIT_THREADS, 2) gang_fit_kernel(FitArgs a) {
   constexpr bool WORDS = OUT != FIT_OUT_NONE;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr size_t STAGE_BYTES = fit_tile_bytes(LW, LN, LS);
   constexpr int LNS = LN + LS;
-  constexpr int STAGES = fit_stages(LW, LN, LS, SCORE);
   unsigned char* s_tile = smem_raw;
-  int64_t* s_req_w = reinterpret_cast<int64_t*>(smem_raw + STAGES * STAGE_BYTES);
+  int64_t* s_req_w = reinterpret_cast<int64_t*>(smem_raw + FIT_STAGES * STAGE_BYTES);
   int32_t* s_req_n = reinterpret_cast<int32_t*>(s_req_w + PODS_PER_CTA * LW);
   uint64_t* s_bar = reinterpret_cast<uint64_t*>(
       (reinterpret_cast<uintptr_t>(s_req_n + PODS_PER_CTA * LNS) + 7) & ~(uintptr_t)7);
-  uint64_t* s_full = s_bar;                 // [STAGES] TMA bytes landed
-  uint64_t* s_empty = s_bar + STAGES;       // [STAGES] every warp is done with the stage
-  uint32_t* s_words_all = reinterpret_cast<uint32_t*>(s_bar + 2 * STAGES);
+  uint64_t* s_full = s_bar;                 // [FIT_STAGES] TMA bytes landed
+  uint64_t* s_empty = s_bar + FIT_STAGES;   // [FIT_STAGES] every warp is done with the stage
+  uint32_t* s_words_all = reinterpret_cast<uint32_t*>(s_bar + 2 * FIT_STAGES);
 
   const uint32_t tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   uint32_t* s_words = s_words_all + wid * PODS_PER_WARP * 32;   // per pod: the 32-word (1024-node) bitmap line being assembled
@@ -322,7 +259,7 @@ __global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MIN
   const uint32_t tile_hi = min(n_tiles, (n_lines * (piece + 1) / npieces) * TILES_PER_LINE);
 
   if (tid == 0) {
-    for (int st = 0; st < STAGES; ++st) {
+    for (int st = 0; st < FIT_STAGES; ++st) {
       mbar_init(&s_full[st], 1);
       mbar_init(&s_empty[st], FIT_WARPS);
     }
@@ -364,12 +301,9 @@ __global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MIN
   // every consumer warp has released the stage (`empty`), and issues the TMA bulk copies that
   // complete on `full`.  Consumers never meet at a CTA-wide barrier during the sweep.
   if (wid == FIT_WARPS) {
-#if BS_FIT_EXP == 5
-    return;
-#endif
     if (lane == 0) {
       for (uint32_t tile = tile_lo; tile < tile_hi; ++tile) {
-        const uint32_t st = (tile - tile_lo) % STAGES, use = (tile - tile_lo) / STAGES;
+        const uint32_t st = (tile - tile_lo) % FIT_STAGES, use = (tile - tile_lo) / FIT_STAGES;
         if (use > 0) mbar_wait(&s_empty[st], (use - 1) & 1);
         issue(tile, st);
       }
@@ -398,15 +332,10 @@ __global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MIN
 #pragma unroll
     for (int d = 0; d < LNS; ++d) rqn[r][d] = s_req_n[(wid * PODS_PER_WARP + r) * LNS + d];
   }
-  const uint32_t slab0 = smem_u32(smem_raw + fit_smem_front(LW, LN, LS, STAGES)) + wid * (uint32_t)(FIT_NB * fit_slab_bytes());
-  int64_t* srow = SCORE ? a.score + (size_t)wpod0 * a.score_pitch : nullptr;
-#ifdef BS_FIT_L2HINT
-  const uint64_t l2pol = l2_evict_first_policy();
-#endif
 
   // Consumers: a warp releases a stage by arriving on its `empty` mbarrier and may run up to
-  // STAGES-1 tiles ahead of the slowest warp.
-  uint32_t stage = 0, phase = 0, sb = 0, nseg = 0;
+  // FIT_STAGES-1 tiles ahead of the slowest warp.
+  uint32_t stage = 0, phase = 0;
   ColBits colnext[PODS_PER_WARP];   // class bits are fetched one tile ahead (their L2 latency stays off the tile's critical path)
 #pragma unroll
   for (int r = 0; r < PODS_PER_WARP; ++r) colnext[r] = __ldg(a.classfit + coff[r] + min(tile_lo, n_tiles - 1) * 32);
@@ -418,54 +347,12 @@ __global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MIN
       colbits[r] = colnext[r];
       colnext[r] = __ldg(a.classfit + coff[r] + tnext * 32);
     }
-#if BS_FIT_EXP != 5
     mbar_wait(&s_full[stage], phase);
-#endif
     const int64_t* tlw = reinterpret_cast<const int64_t*>(s_tile + stage * STAGE_BYTES);
     const int32_t* tln = reinterpret_cast<const int32_t*>(s_tile + stage * STAGE_BYTES + (size_t)LW * NODE_TILE * 8);
     const uint32_t node_base = tile * NODE_TILE;
     const uint32_t wbase = (tile % TILES_PER_LINE) * TILE_WORDS;
-    // the tile in store segments of FIT_SEG nodes: each goes to the next of the warp's FIT_NB staging slabs and
-    // leaves as PODS_PER_WARP bulk stores (one per matrix row) while the following segment is computed
-#pragma unroll 1
-    for (int sg = 0; sg < NODE_TILE / FIT_SEG; ++sg) {
-      const uint32_t slab = slab0 + sb * (uint32_t)fit_slab_bytes();
-#ifdef BS_FIT_STG
-      constexpr bool STAGE = false;
-#else
-      constexpr bool STAGE = SCORE;
-#endif
-      if (STAGE && nseg >= (uint32_t)FIT_NB) {
-        if (lane == 0) bulk_wait_read<FIT_NB - 1>();   // the bulk stores that last read this slab are done with it
-        __syncwarp();
-      }
-      fit_seg<LW, LN, LS, OUT>(a, tlw, tln, rqw, rqn, colbits, slab, s_words, wbase, node_base, lane, sg * SEG_WORDS, best_s, best_n, kb, cnt, wpod0);
-      if (STAGE) {
-        fence_async_smem();
-        __syncwarp();
-        if (lane == 0) {
-          // row segments: FIT_SEG scores, or what is left of the row (pitch is even: 16-byte sizes)
-          const uint32_t col0 = node_base + sg * FIT_SEG;
-#if BS_FIT_EXP == 1    // (experiment 1: staging stores without the bulk stores)
-          if (false) {
-#else
-          if (col0 < (uint32_t)a.score_pitch) {
-#endif
-            const uint32_t cols = min((uint32_t)FIT_SEG, (uint32_t)a.score_pitch - col0);
-#pragma unroll
-            for (int r = 0; r < PODS_PER_WARP; ++r)
-#ifdef BS_FIT_L2HINT
-              tma_bulk_s2g_hint(srow + (size_t)r * a.score_pitch + col0, slab + r * (FIT_SEG * 8), cols * 8, l2pol);
-#else
-              tma_bulk_s2g(srow + (size_t)r * a.score_pitch + col0, slab + r * (FIT_SEG * 8), cols * 8);
-#endif
-          }
-          bulk_commit();
-        }
-        ++nseg;
-        if (++sb == FIT_NB) sb = 0;
-      }
-    }
+    fit_tile<LW, LN, LS, OUT>(a, tlw, tln, rqw, rqn, colbits, s_words, wbase, node_base, lane, best_s, best_n, kb, cnt, wpod0);
     if (LN > 0) {
       // a tile's best key beats the running best iff key >= (best_s + 1) << KEY_BITS: strictly greater score
       // (an equal score in a later tile loses to the earlier node)
@@ -492,18 +379,13 @@ __global__ void __launch_bounds__(FIT_THREADS, OUT == FIT_OUT_SCORE ? BS_FIT_MIN
         for (int r = 0; r < PODS_PER_WARP; ++r) {
           const uint32_t w = s_words[r * 32 + lane];
           cnt[r] += __popc(w);
-#if BS_FIT_EXP != 4
           if (want_bitmap) a.fit_bitmap[(size_t)(wpod0 + r) * a.bitmap_pitch + line * 32 + lane] = w;
-#endif
         }
       }
     }
     __syncwarp();                                   // the ballot slab is rewritten by the next tile
-    if (++stage == STAGES) { stage = 0; phase ^= 1; }
+    if (++stage == FIT_STAGES) { stage = 0; phase ^= 1; }
   }
-#ifndef BS_FIT_STG
-  if (SCORE && lane == 0) bulk_wait_read<0>();      // the slabs must outlive their bulk reads
-#endif
 
   // per-pod reductions across the warp: best = max score, lowest node on ties
 #pragma unroll
@@ -543,9 +425,7 @@ static __global__ void fit_unpack_kernel(const unsigned long long* __restrict__ 
   best_node[p] = (int32_t)(~(uint32_t)v);
   best_score[p] = (int64_t)(v >> 32) - 1;
 }
-#ifndef BS_FIT_TAIL_SPLIT
-#define BS_FIT_TAIL_SPLIT 8   // pieces a tail unit is cut into at most (1 = off)
-#endif
+constexpr uint32_t FIT_TAIL_SPLIT = 8;   // pieces a tail unit is cut into at most
 
 }  // namespace bsk
 

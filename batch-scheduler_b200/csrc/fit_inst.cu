@@ -14,7 +14,7 @@ namespace {
 
 template <int LW, int LN, int LS, int OUT>
 cudaError_t launch_fit_t(const FitArgs& a0, uint32_t units, cudaStream_t s, uint32_t* launches, cudaEvent_t ev_a, cudaEvent_t ev_b) {
-  const size_t smem = gang_fit_smem_bytes(LW, LN, LS, OUT == FIT_OUT_SCORE);
+  const size_t smem = gang_fit_smem_bytes(LW, LN, LS);
   // per launch, not cached: the attribute is per device and one process may drive several GPUs
   cudaError_t er = cudaFuncSetAttribute(gang_fit_kernel<LW, LN, LS, OUT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         (int)smem);
@@ -25,7 +25,7 @@ cudaError_t launch_fit_t(const FitArgs& a0, uint32_t units, cudaStream_t s, uint
   // Tail balance (FitArgs): whole waves of resident CTA slots run full-range units; the units of the last,
   // partial wave are cut into node-range pieces so that every SM gets a share of it.  Narrow shapes only
   // (the packed best needs scores below 2^31).
-  if (LN > 0 && BS_FIT_TAIL_SPLIT > 1 && a.best_packed && units) {
+  if (LN > 0 && a.best_packed && units) {
     int per_sm = 0, dev = 0, sms = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gang_fit_kernel<LW, LN, LS, OUT>, FIT_THREADS, smem) == cudaSuccess &&
         cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess &&
@@ -33,7 +33,7 @@ cudaError_t launch_fit_t(const FitArgs& a0, uint32_t units, cudaStream_t s, uint
       const uint32_t slots = (uint32_t)per_sm * (uint32_t)sms;
       const uint32_t n_tiles = a.Npad / NODE_TILE, n_lines = (n_tiles + TILES_PER_LINE - 1) / TILES_PER_LINE;
       const uint32_t n_full = units / slots * slots, tail = units - n_full;
-      const uint32_t split = std::min<uint32_t>(BS_FIT_TAIL_SPLIT, n_lines);
+      const uint32_t split = std::min(FIT_TAIL_SPLIT, n_lines);
       if (tail && split > 1 && tail * 10 < slots * 9) {   // a nearly full last wave is left alone
         a.n_full = n_full;
         a.tail_split = split;
@@ -78,8 +78,8 @@ FitFn BS_CAT(fit_lookup_slice, BS_FIT_SLICE)(uint32_t LW, uint32_t LN, uint32_t 
 #if BS_FIT_SLICE == 0
   if (LN != 0 || LS != 0) return nullptr;
   switch (LW) {
-#ifndef BS_FIT_MINIMAL
     case 4: return pick<4, 0, 0>(score);
+    case 5: return pick<5, 0, 0>(score);
     case 6: return pick<6, 0, 0>(score);
     case 7: return pick<7, 0, 0>(score);
     case 8: return pick<8, 0, 0>(score);
@@ -91,18 +91,11 @@ FitFn BS_CAT(fit_lookup_slice, BS_FIT_SLICE)(uint32_t LW, uint32_t LN, uint32_t 
     case 14: return pick<14, 0, 0>(score);
     case 15: return pick<15, 0, 0>(score);
     case 16: return pick<16, 0, 0>(score);
-#endif
-    case 5: return pick<5, 0, 0>(score);
   }
   return nullptr;
 #else
   constexpr int N = BS_FIT_SLICE;
   if (LN != (uint32_t)N || !fit_variant_exists(LW, LN, LS)) return nullptr;
-#ifdef BS_FIT_MINIMAL   // development builds: only the shapes of the bench workload
-  if (N == 3 && LW == 0 && LS == 2) return pick<0, N, 2>(score);
-  if (N == 3 && LW == 2 && LS == 0) return pick<2, N, 0>(score);
-  return nullptr;
-#else
   const uint32_t key = LW * 8 + LS;
   switch (key) {
 #define BS_CASE(lw, ls)                                                        \
@@ -113,7 +106,6 @@ FitFn BS_CAT(fit_lookup_slice, BS_FIT_SLICE)(uint32_t LW, uint32_t LN, uint32_t 
 #undef BS_CASE
   }
   return nullptr;
-#endif
 #endif
 }
 

@@ -3,7 +3,7 @@
 instructions: one trip = 4 nodes per lane x PODS_PER_WARP pods) and writes profiles/sass_ops_r2.json, the
 op counts behind the decisions-only instruction roofline in bench.py (SURVEY 8(d) R2).
 
-    python profiles/tools/sass_count.py [--lib batch-scheduler_b200/libbsched.so] [--kernel ILi0ELi3ELi2ELb0E]
+    python profiles/tools/sass_count.py [--lib batch-scheduler_b200/libbsched.so] [--kernel ILi0ELi3ELi2ELi0E]
                                         [--ppw 4] [--dump profiles/sass_gang_fit_r2.txt]
 
 Pipe classes (sm_100a, as ncu groups them): the integer ALU pipe takes add/logic/shift/compare/select/
@@ -39,7 +39,9 @@ def classify(mn):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--lib", default=os.path.join(ROOT, "batch-scheduler_b200", "libbsched.so"))
-    ap.add_argument("--kernel", default="ILi0ELi3ELi2ELb0E", help="substring of the mangled gang_fit_kernel instance")
+    ap.add_argument("--kernel", default="ILi0ELi3ELi2ELi0E",
+                    help="substring of the mangled gang_fit_kernel instance (default: <0,3,2,FIT_OUT_NONE>, the bench shape "
+                         "in decisions-only mode)")
     ap.add_argument("--ppw", type=int, default=4)
     ap.add_argument("--marks-per-pair", type=int, default=4, help="VIADDMNMX per pair: (LN - 1) + LS, 4 for the bench shape (0,3,2)")
     ap.add_argument("--dump", default=None)
@@ -98,9 +100,9 @@ def main():
            "alu_pipe_ops_per_pair": by_class.get("alu", 0) / pairs, "fma_pipe_ops_per_pair": by_class.get("fma", 0) / pairs,
            "lsu_ops_per_pair": by_class.get("lsu", 0) / pairs, "by_class": by_class,
            "by_mnemonic": dict(sorted(by_mn.items(), key=lambda kv: -kv[1])),
-           "note": "static count of the innermost loop that holds the lane arithmetic; with FIT_SEG = 128 nodes the 4-word "
-                   "compute loop is fully unrolled into the segment loop, so the count INCLUDES the per-segment staging overhead "
-                   "(fence, bulk-store issue) in score mode; per-tile / per-sweep instructions outside it are not counted"}
+           "note": "static count of the innermost loop that holds the lane arithmetic (one trip = 4 nodes per lane x "
+                   "PODS_PER_WARP pods); in score mode it includes the streaming score stores and their bounds checks; "
+                   "per-tile / per-sweep instructions outside it are not counted"}
     with open(a.out, "w") as f:
         json.dump(out, f, indent=1)
     print(json.dumps({k: out[k] for k in ("kernel", "instructions_in_loop", "pairs_per_trip", "issue_ops_per_pair",
